@@ -4,6 +4,7 @@
   python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (CUDA, through the C ABI)
   python bench.py --impl reference [...]                         reference arm: the CPU path on the box's host cores
   python bench.py --mode build|sharded|headline [...]            one leg only (default --mode auto, below)
+  python bench.py --dump-outputs DIR [...]                       also write the last timed search step's results as DIR/*.npy
 
 A "step" = one pass of the hot path (Hnsw::search, lib.rs:352-383) over one batch of synthetic queries.
 
@@ -29,11 +30,13 @@ so no L2 flush is needed between iterations.  torch is plumbing only: device buf
 """
 import argparse
 import ctypes as C
+import functools
 import hashlib
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -158,13 +161,25 @@ def permute_points(pts, ids):
 
 
 def cache_dir():
-    d = os.environ.get("IDB_CACHE", os.path.join(ROOT, "gpurun_cache"))
+    """IDB_CACHE, else a per-user directory under the system temp dir: the tree bench.py runs from may be read-only."""
+    d = os.environ.get("IDB_CACHE") or os.path.join(tempfile.gettempdir(), f"idb_bench_cache_{os.getuid()}")
     os.makedirs(d, exist_ok=True)
     return d
 
 
-def graph_cache_path(n, dim, data, data_seed, M, efc, seed):
-    key = f"{n}-{dim}-{data}-{data_seed}-{M}-{efc}-{seed}-v3"
+@functools.lru_cache(maxsize=None)
+def file_digest(path):
+    h = hashlib.sha1()
+    with open(path, "rb") as f:
+        for block in iter(lambda: f.read(1 << 22), b""):
+            h.update(block)
+    return h.hexdigest()
+
+
+def graph_cache_path(n, dim, data, data_seed, M, efc, seed, builder):
+    """`builder` is the binary that builds the graph (the CUDA library, or the oracle's for --graph oracle).  Its digest is part of
+    the key, so a cached graph is only reused by the same build of the code that made it, whichever checkout runs bench.py."""
+    key = f"{n}-{dim}-{data}-{data_seed}-{M}-{efc}-{seed}-{os.path.basename(builder)}-{file_digest(builder)}-v4"
     return os.path.join(cache_dir(), "graph_" + hashlib.sha1(key.encode()).hexdigest()[:16] + ".npz")
 
 
@@ -195,14 +210,22 @@ def build_graph_with_tool(pts, M, efc, ef, seed, device):
 
 def obtain_graph(pts, n, dim, data, data_seed, M, efc, ef, seed, device, use_abi, no_cache=False, by="gpu"):
     """(points in PointId order, zero, upper, ids).  The graph is the GPU Builder::build's (deterministic in the seed): built
-    in-process when the caller is the CUDA arm (use_abi), else by the C++ tool; cached under gpurun_cache/ (git-ignored).
+    in-process when the caller is the CUDA arm (use_abi), else by the C++ tool; cached under cache_dir() (graph_cache_path).
     by="oracle" (--graph oracle): the reference algorithm's own threaded CPU build (lib.rs:313-318) instead — BASELINE configs[1]'s
     "reference-built graph" to the letter; minutes of host time at 1M points, so it is not the default."""
-    cp = graph_cache_path(n, dim, data, data_seed, M, efc, seed)
     if by == "oracle":
-        cp = cp.replace("graph_", "graph_oracle_")
+        from oracle import oracle as O
+
+        builder = O.build_lib()
         use_abi = False
-    if os.path.exists(cp) and not no_cache:
+    elif use_abi:
+        from instant_distance_b200 import _abi
+
+        builder = _abi.LIB_PATH
+    else:
+        builder = os.path.join(os.path.dirname(TOOL), "libinstant_distance_b200.so")  # the library the tool loads
+    cp = graph_cache_path(n, dim, data, data_seed, M, efc, seed, builder) if os.path.exists(builder) else None
+    if cp and os.path.exists(cp) and not no_cache:
         try:
             z = np.load(cp)
             got = permute_points(pts, z["ids"]), z["zero"], [z[f"u{i}"] for i in range(int(z["n_upper"]))], z["ids"]
@@ -229,6 +252,7 @@ def obtain_graph(pts, n, dim, data, data_seed, M, efc, ef, seed, device, use_abi
             ids = None
     else:
         ids = None
+    stand_in = ids is None and by != "oracle"  # the oracle builds in place of the GPU build: not cached under the library's key
     if ids is None:
         from oracle import oracle as O
 
@@ -241,7 +265,7 @@ def obtain_graph(pts, n, dim, data, data_seed, M, efc, ef, seed, device, use_abi
             GRAPH_HOW["by"] = GRAPH_HOW["sharded"] = "oracle (reference algorithm, threaded CPU build): no GPU was available to this arm"
         log("graph built by the oracle (CPU) — NOT the GPU build's graph")
     log(f"graph built in {time.time() - t:.1f}s (setup, untimed)")
-    if not no_cache:
+    if cp and not no_cache and not stand_in:
         try:
             tmp = cp[:-4] + f".{os.getpid()}.tmp.npz"  # written whole, then renamed: a reader never sees a partial file
             np.savez(tmp, ids=ids, zero=zero, n_upper=len(upper), **{f"u{i}": u for i, u in enumerate(upper)})
@@ -308,6 +332,26 @@ def cpu_qps(search_fn, batches, warm, timed):
         search_fn(b)
     dt = time.perf_counter() - t0
     return sum(len(b) for b in batches[warm:warm + timed]) / dt, dt
+
+
+DUMP_BYTES = 64_000_000  # all files of one dump, .npy headers included
+NPY_HEADER = 128  # bytes of an .npy (v1.0) header for these shapes
+
+
+def dump_outputs(d, outputs):
+    """--dump-outputs: the last timed step's results (one row per query) as d/<name>.npy — ids and lengths as float64 (exact),
+    distances as float32 — so that two builds can be compared output for output.  Beyond DUMP_BYTES in all, a fixed seeded
+    sample of rows is written instead, with the sampled row numbers as rows.npy."""
+    out = {k: v.astype(np.float32 if v.dtype == np.float32 else np.float64) for k, v in outputs.items()}
+    n = len(out["ids"])
+    row_bytes = sum(v.nbytes for v in out.values()) // n
+    if n * row_bytes + NPY_HEADER * len(out) > DUMP_BYTES:
+        m = (DUMP_BYTES - NPY_HEADER * (len(out) + 1)) // (row_bytes + 8)  # (+ 8: the row number in rows.npy)
+        rows = np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+        out = {**{k: v[rows] for k, v in out.items()}, "rows": rows.astype(np.float64)}
+    os.makedirs(d, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(d, k + ".npy"), v)
 
 
 def pinned(nbytes, dtype, shape):
@@ -420,6 +464,9 @@ def leg_search(a, rank, local_rank, world, full=True):
 
     lanes = a.lanes
     dev_ms, clocks, launches = device_arm(lanes)
+    last = (total - 1) % lanes  # the last timed step's results, before the sweep and the isolated launches reuse the buffers
+    outputs = {"ids": d_ids[last].cpu().numpy().view(np.uint32), "distances": d_dist[last].cpu().numpy(),
+               "lengths": d_len[last].cpu().numpy().view(np.uint32)}
     qps = world * nq * a.steps / (dev_ms / 1e3)
     sweep = None
     if a.sweep and full:
@@ -447,6 +494,7 @@ def leg_search(a, rank, local_rank, world, full=True):
                      "kernel_ms": k_ms, "kernel_ms_note": f"timed region / launches, {lanes} launches in flight (successive launches overlap at the batch boundary)",
                      "kernel_ms_isolated": float(np.mean(iso_ms)), "frac_isolated": alg / (float(np.mean(iso_ms)) / 1e3) / 1e9 / peak,
                      "algorithmic_bytes_per_launch": alg, "peak_source": peak_src},
+        "outputs": outputs,
     }
     if a.n == 1_000_000 and a.dim == 128 and a.batch == 10_000 and a.data == "sift":
         res["roofline"]["traffic"], res["roofline"]["traffic_source"] = ncu_traffic()
@@ -513,10 +561,10 @@ def leg_search(a, rank, local_rank, world, full=True):
                     and (o_len == last_ids["len"][:sample]).all() and (o_cnt == g_cnt).all())
         if not same:
             log("PARITY FAILURE: GPU results differ from the oracle on the same graph")
-        batches = [q[:sample] for q in host_q[:8]]
-        v, dt = cpu_qps(lambda b: ox.search(b, ef_search=ef, k=K, threads=T), batches, 3, len(batches) - 3)
+        batches = [q[:sample] for q in host_q]
+        v, dt = cpu_qps(lambda b: ox.search(b, ef_search=ef, k=K, threads=T), batches, a.warmup, a.steps)
         res["cpu_baseline"] = {"value": v, "unit": "queries/s", "cores": T, "kind": "port",
-                               "sample": f"{len(batches) - 3} passes of {sample} queries after 3 warm passes ({dt:.1f} s), same graph, ef_search={ef}, "
+                               "sample": f"{a.steps} passes of {sample} queries after {a.warmup} warm passes ({dt:.1f} s), same graph, ef_search={ef}, "
                                          f"{T} threads (one Search per thread); GPU ids/distances/lengths/counters identical to the oracle's: {same}"}
         res["parity_ok"] = same
     ix.close()
@@ -610,6 +658,7 @@ def leg_sharded(a, rank, local_rank, world, full=True):
     sampler.stop()
     qps = nq * a.steps / (dev_ms / 1e3)
     launches = a.steps * (2 * per + (1 if per > 1 else 0) + 2)  # per shard K1 + retry; pre-merge; all-gather; merge
+    outputs = {"ids": d_ids.cpu().numpy().view(np.uint32), "distances": d_dist.cpu().numpy(), "lengths": d_len.cpu().numpy().view(np.uint32)}
 
     # K1 of the rank's first sub-index, isolated, for the roofline of the dominant kernel
     shards[0].search_device(dq_pool[0].data_ptr(), nq, a.ef, K, d_ids.data_ptr(), d_dist.data_ptr(), d_len.data_ptr())
@@ -644,7 +693,7 @@ def leg_sharded(a, rank, local_rank, world, full=True):
                      "traffic": None, "kernel": "search_kernel (K1) of one sub-index, isolated launch", "kernel_ms": k_ms,
                      "algorithmic_bytes_per_launch": alg, "peak_source": peak_src,
                      "share_of_step": per * k_ms / (dev_ms / a.steps)},
-        "build_s_per_rank": t_build,
+        "build_s_per_rank": t_build, "outputs": outputs,
     }
     if not protocol_ok:
         log("PROTOCOL FAILURE: the fused sharded search differs from the host statement of the protocol")
@@ -661,16 +710,15 @@ def leg_sharded(a, rank, local_rank, world, full=True):
             _abi.check(L.idb_sharded_search_batch_f32_multi(hs, len(shards), comm._h, _abi.ptr(hq[s % 2], C.c_float), nq, a.ef, K,
                                                             _abi.ptr(hid, C.c_uint32), _abi.ptr(hds, C.c_float), _abi.ptr(hln, C.c_uint32)))
 
-        n_e2e = max(3, a.steps // 2)
-        for s in range(2):
+        for s in range(a.warmup):
             e2e_step(s)
         barrier(world)
         t0 = time.perf_counter()
-        for s in range(n_e2e):
+        for s in range(a.steps):
             e2e_step(s)
         e2e_s = reduce_max(time.perf_counter() - t0, world)
-        res["e2e"] = {"value": nq * n_e2e / e2e_s, "unit": "queries/s", "h2d_bytes_per_step": nq * a.dim * 4,
-                      "d2h_bytes_per_step": nq * K * 8 + nq * 4, "steps": n_e2e}
+        res["e2e"] = {"value": nq * a.steps / e2e_s, "unit": "queries/s", "h2d_bytes_per_step": nq * a.dim * 4,
+                      "d2h_bytes_per_step": nq * K * 8 + nq * 4, "steps": a.steps}
         # parity of one sub-index against the oracle on that sub-index's graph (rank 0's first)
         if rank == 0 and not a.skip_cpu_baseline:
             from oracle import oracle as O
@@ -735,16 +783,17 @@ def leg_build(a, local_rank):
     d_len = torch.empty((nq,), dtype=torch.int32, device="cuda")
     ix.set_profiling(True)
     k_ms, alg = [], []
-    for s in range(3 + 5):
+    for s in range(a.warmup + a.steps):
         ix.search_device(dq[s % 4].data_ptr(), nq, ef_s, K, d_ids.data_ptr(), d_dist.data_ptr(), d_len.data_ptr())
         ms, _ = ix.last_kernel_ms()
-        if s >= 3:
+        if s >= a.warmup:
             k_ms.append(ms)
             alg.append(float(algorithmic_bytes(ix.last_counters(nq), a.dim, a.M, K).sum()))
     peak, _ = measured_peaks()
     res["search"] = {"value": nq / (float(np.mean(k_ms)) / 1e3), "unit": "queries/s", "batch": nq, "ef_search": ef_s, "recall_at_10": rec_s,
                      "kernel_ms": float(np.mean(k_ms)), "k1_frac": float(np.mean(alg)) / (float(np.mean(k_ms)) / 1e3) / 1e9 / peak,
-                     "what": "K1 launches of one 10k-query batch each (device-resident, isolated, 5 timed after 3 warm), on the graph built above"}
+                     "what": f"K1 launches of one {nq}-query batch each (device-resident, isolated, {a.steps} timed after {a.warmup} warm), "
+                             "on the graph built above"}
     del dq, d_ids, d_dist, d_len
     if not a.skip_cpu_baseline:
         from oracle import oracle as O
@@ -789,7 +838,9 @@ def run_reference(a, rank, world):
         ix = O.from_graph(O.Graph(p, zero, upper, a.M, a.ef))
         sample = min(a.batch, a.ref_sample)
         batches = [gen(sample, a.dim, 5000 + s)[:sample] for s in range(a.warmup + a.steps)]
-        qps, dt = cpu_qps(lambda b: ix.search(b, ef_search=a.ef, k=K, threads=T), batches, a.warmup, a.steps)
+        last = []
+        qps, dt = cpu_qps(lambda b: last.append(ix.search(b, ef_search=a.ef, k=K, threads=T)), batches, a.warmup, a.steps)
+        outputs = dict(zip(("ids", "distances", "lengths"), last[-1]))
         cfg = search_config(a, 1, "headline")
         metric = "batched QPS at recall@10>=0.95 (1M x 128 f32)"
         desc = f"{sample} queries per step x {a.steps} steps after {a.warmup} warm steps, same graph/ef, {T} threads, one Search per thread"
@@ -816,7 +867,12 @@ def run_reference(a, rank, world):
                 keys.append(kk)
             return np.sort(np.concatenate(keys, axis=1), axis=1)[:, :K]
 
-        qps, dt = cpu_qps(search_all, batches, a.warmup, a.steps)
+        last = []
+        qps, dt = cpu_qps(lambda b: last.append(search_all(b)), batches, a.warmup, a.steps)
+        if a.dump_outputs:
+            from instant_distance_b200.sharded import merge_keys  # (host code only: the CUDA library stays unloaded)
+
+            outputs = dict(zip(("ids", "distances", "lengths"), merge_keys(last[-1][None], K)))
         cfg = sharded_config(a, world)
         metric = "batched QPS, 10M x 128 f32 in 8 PointId-range sub-indexes (BASELINE configs[4])"
         desc = (f"{sample} queries per step x {a.steps} steps after {a.warmup} warm steps, each searched on all {N_SUB} sub-indexes and merged on the "
@@ -828,6 +884,8 @@ def run_reference(a, rank, world):
         "config": cfg, "cpu_baseline": {"value": qps, "unit": "queries/s", "cores": T, "kind": "port", "sample": desc},
         "e2e": {"value": qps, "unit": "queries/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
 
 
@@ -862,8 +920,12 @@ def main():
     ap.add_argument("--sweep", action="store_true", help="also time 1..4 lanes / callers (reported under `sweep`)")
     ap.add_argument("--build-reps", type=int, default=2)
     ap.add_argument("--build-cpu-sample", type=int, default=100_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the ids, distances and lengths of the last timed search step as DIR/<name>.npy")
     a = ap.parse_args()
     a.warmup = max(a.warmup, 3)  # timing rule: at least 3 untimed warm-up steps
+    if a.dump_outputs and a.impl == "ours" and a.mode == "build":
+        ap.error("--dump-outputs needs a search mode (--mode auto, headline or sharded)")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -887,13 +949,14 @@ def main():
     common = {"n_gpus": world, "steps": a.steps, "warmup": a.warmup, "higher_is_better": True, "vs_baseline": None, "dtype": "f32",
               "data": "synthetic"}
 
-    out = None
+    out = outputs = None
     if mode == "build":
         res = leg_build(a, local_rank)
         out = {**res, **common, "scaling": "weak"}
     elif mode == "headline":
         t_leg = time.time()
         h = leg_search(a, rank, local_rank, world)
+        outputs = h.get("outputs")
         log(f"headline leg took {time.time() - t_leg:.1f}s")
         line = {"metric": "batched QPS at recall@10>=0.95 (1M x 128 f32)", "value": h["value"], "unit": "queries/s", **common,
                 "ms_per_step": h["ms_per_step"], "scaling": "weak"}
@@ -927,7 +990,7 @@ def main():
                      "cpu_baseline": h.get("cpu_baseline"), "clocks": h["clocks"]})
 
         def uniform_leg():
-            ua = argparse.Namespace(**{**vars(a), "data": "uniform", "steps": min(a.steps, 10), "graph": "gpu"})
+            ua = argparse.Namespace(**{**vars(a), "data": "uniform", "graph": "gpu"})
             u = leg_search(ua, rank, local_rank, world, full=False)
             return {"value": u["value"], "unit": "queries/s", "recall_at_10": u["recall_at_10"], "ef_search": u["ef_search"],
                     "k1_frac": u["roofline"]["frac"]}
@@ -947,12 +1010,13 @@ def main():
         out = line
     else:  # sharded
         s = leg_sharded(a, rank, local_rank, world)
+        outputs = s.get("outputs")
         line = {"metric": "batched QPS, 10M x 128 f32 in 8 PointId-range sub-indexes (BASELINE configs[4])", "value": s["value"], "unit": "queries/s",
                 **common, "ms_per_step": s["ms_per_step"], "scaling": "strong",
                 "strong_scaling_note": "the 1-GPU point of this curve is `sharded.value` of the --gpus 1 line (same 8 sub-indexes on one GPU); that line's "
                                        "primary value is configs[1], as the bench contract requires at N=1"}
         if world > 1 and a.mode == "auto" and not a.skip_secondary:
-            ra = argparse.Namespace(**{**vars(a), "steps": min(a.steps, 10), "graph": "gpu"})
+            ra = argparse.Namespace(**{**vars(a), "graph": "gpu"})
             r = leg_search(ra, rank, local_rank, world, full=False)
             line["replicas"] = {"what": "configs[1] with the 1M index replicated per GPU and the queries sharded (no collective)", "value": r["value"],
                                 "unit": "queries/s", "k1_frac": r["roofline"]["frac"], "recall_at_10": r["recall_at_10"]}
@@ -978,6 +1042,8 @@ def main():
     if world > 1:
         dist.destroy_process_group()  # (before the JSON line: NCCL's own log lines may share stdout)
     if rank == 0:
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, outputs)
         print(json.dumps(out), flush=True)
 
 

@@ -4,6 +4,7 @@ for real."""
 import json
 import sys
 
+import numpy as np
 import pytest
 
 import bench
@@ -86,3 +87,72 @@ def test_a_failing_secondary_leg_does_not_take_the_headline_down(cpu_bench, caps
 def test_skip_secondary_prints_the_headline_only(cpu_bench, capsys):
     line = cpu_bench(["--skip-secondary"], capsys)
     assert "sharded" not in line and "uniform" not in line and "build" not in line and line["roofline"]["bound"] == "hbm"
+
+
+def test_dump_outputs_writes_the_last_steps_results(cpu_bench, capsys, monkeypatch, tmp_path):
+    rng = np.random.default_rng(1)
+    ids = rng.integers(0, 1 << 20, (1000, 10)).astype(np.uint32)
+    ids[3, 7:] = 0xFFFFFFFF
+    outs = {"ids": ids, "distances": rng.random((1000, 10), dtype=np.float32), "lengths": np.full(1000, 10, np.uint32)}
+    monkeypatch.setattr(bench, "leg_search", lambda *a_, **k_: {**fake_search(*a_, **k_), "outputs": outs})
+    cpu_bench(["--skip-secondary", "--dump-outputs", str(tmp_path / "all")], capsys)
+    got = {k: np.load(tmp_path / "all" / f"{k}.npy") for k in outs}
+    assert got["ids"].dtype == np.float64 and (got["ids"] == ids).all() and got["ids"][3, 9] == 0xFFFFFFFF
+    assert got["distances"].dtype == np.float32 and got["distances"].tobytes() == outs["distances"].tobytes()
+    assert got["lengths"].dtype == np.float64 and (got["lengths"] == 10).all()
+    assert not (tmp_path / "all" / "rows.npy").exists()
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 20_000)  # over the cap: the same seeded sample of rows on every run
+    for d in ("s1", "s2"):
+        cpu_bench(["--skip-secondary", "--dump-outputs", str(tmp_path / d)], capsys)
+    rows = np.load(tmp_path / "s1" / "rows.npy")
+    assert (rows == np.load(tmp_path / "s2" / "rows.npy")).all() and 0 < len(rows) < 1000
+    assert sum(f.stat().st_size for f in (tmp_path / "s1").iterdir()) <= 20_000
+    assert (np.load(tmp_path / "s1" / "ids.npy") == ids[rows.astype(np.int64)]).all()
+
+
+def test_dump_outputs_is_refused_where_there_is_no_search_step(cpu_bench, capsys, tmp_path):
+    with pytest.raises(SystemExit):
+        cpu_bench(["--mode", "build", "--dump-outputs", str(tmp_path)], capsys)
+
+
+@pytest.fixture
+def oracle_graphs(monkeypatch, oracle):
+    """bench.obtain_graph replaced by a single-threaded oracle build, remembered by data seed for the expected results."""
+    graphs = {}
+
+    def obtain(pts, n, dim, data, data_seed, M, efc, ef, seed, *_, **__):
+        ix, ids = oracle.build(pts, M=M, ef_construction=efc, ef_search=ef, seed=seed, threads=1)
+        g = ix.export()
+        graphs[data_seed] = g, ids
+        return g.points, g.zero, g.upper, ids
+
+    monkeypatch.setattr(bench, "obtain_graph", obtain)
+    return graphs
+
+
+@pytest.mark.parametrize("world", [1, 2])
+def test_reference_arm_dumps_its_last_timed_batch(cpu_bench, capsys, monkeypatch, tmp_path, oracle, oracle_graphs, world):
+    """World 1: the configs[1] path, one graph.  World 2: the configs[4] path, every query on all sub-indexes, merged on the host."""
+    from instant_distance_b200.sharded import merge_keys, pack_keys
+    from tests import datagen
+
+    monkeypatch.setenv("WORLD_SIZE", str(world))
+    argv = ["--impl", "reference", "--n", "1500", "--dim", "12", "--batch", "90", "--shard-n", "400", "--ref-sample-sharded", "70",
+            "--steps", "2", "--warmup", "3", "--dump-outputs", str(tmp_path)]
+    line = cpu_bench(argv, capsys)
+    got = [np.load(tmp_path / f"{k}.npy") for k in ("ids", "distances", "lengths")]
+    search = lambda g, q: oracle.from_graph(oracle.Graph(g.points, g.zero, g.upper, 32, 100)).search(q, ef_search=100, k=10)
+    if world == 1:
+        want = search(oracle_graphs[1][0], datagen.sift_shaped(90, 12, 5000 + 4))  # (3 warm + 2 timed: batch 4 is the last)
+    else:
+        q, keys = datagen.sift_shaped(70, 12, 7000 + 4), []
+        for s in range(bench.N_SUB):
+            g, ids = oracle_graphs[1000 + s]
+            i_, d_, l_ = search(g, q)
+            gid = np.empty(400, dtype=np.uint32)  # PointId -> global row number of the sub-index's input range
+            gid[ids] = np.arange(400 * s, 400 * (s + 1))
+            keys.append(pack_keys(d_, gid[np.minimum(i_, 399)], l_))
+        want = merge_keys(np.stack(keys), 10)
+    assert line["steps"] == 2 and got[1].tobytes() == want[1].tobytes()
+    assert (got[0] == want[0]).all() and (got[2] == want[2]).all()

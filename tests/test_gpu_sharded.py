@@ -56,7 +56,7 @@ def test_sharded_search_world_of_one_three_shards(oracle, k, ef):
     [s_.close() for s_ in shards]
 
 
-@pytest.mark.skipif("_gpu_count() < 2", reason="needs >= 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif("_gpu_count() < 2", reason="needs >= 2 GPUs")
 def test_sharded_search_two_ranks():
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
            "--master-port", "29533", os.path.join(ROOT, "scripts", "sharded_check.py"), "--points", "60000", "--queries", "3000"]
